@@ -474,7 +474,7 @@ class GroupProgram:
                 if e.is_integer() and 1 <= abs(e) <= MAX_FAST_POW:
                     e = int(e)
                     if e > 0:
-                        return f"inflx_powi<{e}>({args[0]})"
+                        return f"inflx_powi<{e}>({args[0]}, {pol})"
                     return f"inflx_powi_neg<{-e}>({args[0]}, {pol})"
                 e2 = 2.0 * e
                 if e2.is_integer() and abs(e2) <= 2 * MAX_FAST_POW:

@@ -153,3 +153,54 @@ ZERO_V10_UNIT = SPECIAL_UNIT.replace(
     "    return (x[0] - x[1])/((x[0])*(x[0]) - 1);", "    return 0;"
 ).replace('random999', 'zero_v10')
 assert "return 0;" in ZERO_V10_UNIT
+
+
+# per-point literal powers (exponents 3, -3, 7, 1.5, -2.5, 3.5, 64) of expressions in x[0], x[1] and
+# args[0]: the generator emits the double-double chains inflx_powi / inflx_powi_neg / inflx_powh /
+# inflx_powh_neg.  With args[0] = 2^300, 2^-300 or 2^345 and x[0] x[1] spanning 2^-20 .. 2^4 on the
+# grid, one grid crosses the overflow, subnormal and zero thresholds of the powers.
+POWER_UNIT = PREAMBLE % (N_PAR, 64) + """
+double V(const double x[], const double args[]){
+    return pow(args[0]*x[0]*x[1], 3) + pow(x[0]*x[1], 64);
+}
+double v00(const double x[], const double args[]){
+    return pow(args[0]*(x[0] + x[1]*x[1]), -3);
+}
+double v01(const double x[], const double args[]){
+    return x[0]*x[1];
+}
+double v10(const double x[], const double args[]){
+    return pow(x[0]*x[1]*args[0], 7) - pow(args[0]*x[0] + x[1], 1.5);
+}
+double v11(const double x[], const double args[]){
+    return pow(args[0]*x[0]*x[1] + x[1], -2.5);
+}
+double grad_norm_squared(const double x[], const double args[]){
+    return pow(args[0]*x[1] + x[0], 3.5);
+}
+double inner_prod(const double x[], const double args[], const double v1[], const double v2[]){
+    const double g00 = 1;
+    const double g11 = 1;
+    return 0.0 + (g00 * v1[0] * v2[0]) + (g11 * v1[1] * v2[1]);
+}
+void v(const double x[], const double args[], double v_out[]){
+    v_out[0] = x[0];
+    v_out[1] = x[1];
+    return;
+}
+void w1(const double x[], const double args[], double v_out[]){
+    v_out[0] = x[1];
+    v_out[1] = x[0];
+    return;
+}
+"""
+POWER_SCALES = (1.0, 2.0**300, 2.0**-300, 2.0**345)
+POWER_EXTENT = (0.001, 4.0, 0.001, 4.0)
+
+# flavour "cr": powers of x[0] alone are evaluated once per grid row, by the same chains
+POWER_ROW_UNIT = POWER_UNIT.replace("random64", "powrow").replace(
+    "return pow(args[0]*x[0]*x[1], 3) + pow(x[0]*x[1], 64);",
+    "return pow(args[0]*x[0], 3) + pow(x[0], 64) + x[1];").replace(
+    "return pow(args[0]*(x[0] + x[1]*x[1]), -3);", "return pow(args[0]*x[0], -3) + x[1];").replace(
+    "return pow(args[0]*x[0]*x[1] + x[1], -2.5);", "return pow(args[0]*x[0], -2.5) + x[1];")
+assert POWER_ROW_UNIT.count(" + x[1];") == 3

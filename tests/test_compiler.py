@@ -160,3 +160,27 @@ def test_piecewise_models_compile():
     art = comp.compile()
     assert "?" in comp.c_source and art.n_parameters == 1
     assert read_artifact_metadata(art.shared_object_path)["flops_per_point"]["potential"] > 7
+
+
+def test_a_cubin_cache_that_cannot_be_written_is_still_used(tmp_path, monkeypatch):
+    """A cache shipped pre-filled in a read-only tree: a cubin it holds is loaded, one it lacks is
+    compiled and returned (and reused within the process) instead of failing on the write."""
+    from inflatox_b200 import compiler
+
+    monkeypatch.setenv("INFLATOX_CACHE_DIR", str(tmp_path))
+    opts = ["--gpu-architecture=sm_100a", "--std=c++17"]
+    src = f'extern "C" __global__ void k(double* p) {{ p[0] = 2.0; }}  // {tmp_path.name}'
+    shipped = nvrtc_compile(src, "k.cu", opts)  # writable: stored
+    assert len(list(tmp_path.glob("*.cubin"))) == 1
+
+    def read_only(*args, **kwargs):
+        raise PermissionError(13, "Permission denied")
+
+    monkeypatch.setattr(compiler.os, "replace", read_only)
+    assert nvrtc_compile(src, "k.cu", opts) == shipped
+    other = src.replace("2.0", "3.0")
+    a = nvrtc_compile(other, "k.cu", opts)
+    assert a and a != shipped
+    assert sorted(p.name for p in tmp_path.iterdir()) == [p.name for p in tmp_path.glob("*.cubin")]
+    assert len(list(tmp_path.glob("*.cubin"))) == 1  # nothing stored, no temporary left behind
+    assert nvrtc_compile(other, "k.cu", opts) == a

@@ -143,3 +143,69 @@ def test_constant_zero_v10_takes_the_special_epilogue_bit_for_bit(params, tmp_pa
         ok = _bit_identical(out[..., k], ref[..., k])
         assert ok.all(), (k, out[..., k][~ok][:4], ref[..., k][~ok][:4])
     assert (np.isinf(out) == np.isinf(ref)).all()
+
+
+def _power_lib(c_text, tmp_path, libm="glibc"):
+    comp = Compiler.__new__(Compiler)
+    comp.nvrtc_opts = list(Compiler.default_nvrtc_flags)
+    comp.libm = libm
+    comp.output_path = str(tmp_path / "model.c")
+    art_path = str(tmp_path / "model.bin")
+    comp.build_artifact(c_text, art_path)
+    lib = rs.open_inflx_dylib(art_path, False)
+    lib.set_devices([0])
+    return lib
+
+
+def _within(name, got, ref, some_finite=True):
+    import cases
+
+    err, fin, nan_mm, inf_mm = cases.rel_err(got, ref)
+    assert nan_mm == 0 and inf_mm == 0, (name, nan_mm, inf_mm)
+    assert (fin.any() or not some_finite) and (err[fin] <= 1e-10).all(), (name, float(err[fin].max(initial=0)))
+
+
+@pytest.mark.parametrize("scale", [1.0, 2.0**300, 2.0**-300, 2.0**345])
+def test_per_point_literal_powers_across_overflow_and_underflow(scale, tmp_path):
+    """GPU twin of the host-emulation test of the same name: per-point x^3, x^-3, x^7, x^1.5,
+    x^-2.5, x^3.5, x^64 (double-double chains with the hardware seeds) of operands one grid carries
+    past the overflow and subnormal thresholds - grid ops, the on-trajectory op and calc_V: NaN / inf
+    masks of the oracle (glibc pow) and every finite value within 1e-10 of it."""
+    from raw_units import POWER_EXTENT, POWER_UNIT
+
+    orc = _RawOracle(POWER_UNIT, str(tmp_path))
+    lib = _power_lib(POWER_UNIT, tmp_path)
+    p = np.array([scale, 1.0, 1.0])
+    ext, n0, n1 = POWER_EXTENT, 97, 131
+    ss = np.array(ext).reshape(2, 2)
+    v = np.zeros((n0, n1))
+    lib.potential_array(v, p, ss)
+    _within("potential_array", v, orc.potential_array(p, n0, n1, ext))
+    _within("hesse_array", lib.hesse_array(np.array([n0, n1]), p, ss), orc.hesse_array(p, n0, n1, ext))
+    out = np.zeros((n0, n1, 6))
+    rs.complete_analysis(lib, p, out, ss, False, 0)
+    _within("complete_analysis", out, orc.complete_analysis(p, n0, n1, ext))
+    rng = np.random.default_rng(64)
+    xs = np.ascontiguousarray(np.stack([rng.uniform(ext[0], ext[1], 777), rng.uniform(ext[2], ext[3], 777)], 1))
+    traj = np.zeros((xs.shape[0], 6))
+    rs.complete_analysis_on_trajectory(lib, p, xs, traj, False, 0)
+    _within("complete_analysis_on_trajectory", traj, orc.complete_analysis_on_trajectory(p, xs))
+    calc_v = np.array([lib.potential(x, p) for x in xs[:64]])
+    _within("calc_V", calc_v, np.array([orc.potential(x, p) for x in xs[:64]]), some_finite=False)
+    if scale == 2.0**345:
+        assert np.isinf(v).any() and np.isfinite(v).any()
+
+
+def test_row_class_literal_powers_in_the_correctly_rounded_flavour(tmp_path):
+    """libm="cr": powers of x[0] alone through the same chains in the row pre-pass, across the
+    thresholds: NaN / inf masks of the oracle and every finite point within 1e-10 of it."""
+    from raw_units import POWER_EXTENT, POWER_ROW_UNIT
+
+    orc = _RawOracle(POWER_ROW_UNIT, str(tmp_path))
+    lib = _power_lib(POWER_ROW_UNIT, tmp_path, libm="cr")
+    ext, n0, n1 = POWER_EXTENT, 101, 37
+    for scale in (1.0, 2.0**300, 2.0**-300, 2.0**345):
+        p = np.array([scale, 1.0, 1.0])
+        out = np.zeros((n0, n1, 6))
+        rs.complete_analysis(lib, p, out, np.array(ext).reshape(2, 2), False, 0)
+        _within(f"complete_analysis scale {scale}", out, orc.complete_analysis(p, n0, n1, ext))
